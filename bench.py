@@ -12,6 +12,9 @@ padded, end-repaired strands  ->  k-mer table, unitigs, links, repeat expansion,
 `e2e`    : the same, with the strands copied from pinned host memory inside the timed region (the call a user makes).
 `roofline`: the hash-insert kernel alone (events right around its launch) against the measured HBM copy peak (MEASURED_PEAKS.json).
 `cli_wall`: `autocycler compress` from process start to both files closed (stage A, CUDA context and file I/O included).
+
+--dump-outputs DIR writes what the last timed step returned (dump_outputs), so that two builds can be compared output for output.
+The bench writes nothing into the tree it runs from: the tree may be read-only.
 """
 import argparse
 import json
@@ -21,6 +24,7 @@ import sys
 import threading
 import time
 
+sys.dont_write_bytecode = True
 ROOT = os.path.dirname(os.path.abspath(__file__))
 sys.path.insert(0, ROOT)
 
@@ -55,6 +59,23 @@ def golden_for(key):
         return json.load(open(os.path.join(ROOT, "tests", "golden", "config_goldens.json")))[key]["sha256"]
     except Exception:
         return None
+
+
+DUMP_GFA_MAX = 15_000_000      # bytes of GFA text dumped as float32: 60 MB, under the 64 MB the dump may take
+
+
+def dump_outputs(directory, gfa, counts):
+    """What the timed path returned in its last step, as float arrays: gfa.npy holds the bytes of input_assemblies.gfa (all of them up
+    to DUMP_GFA_MAX, else that many at positions drawn with a fixed seed from the file's length, in file order) and gfa_size.npy their
+    number; graph_counts.npy holds the k-mers, unitigs, links and total unitig length of the graph."""
+    import numpy as np
+    os.makedirs(directory, exist_ok=True)
+    text = np.frombuffer(bytes(gfa), dtype=np.uint8)
+    if text.size > DUMP_GFA_MAX:
+        text = text[np.sort(np.random.default_rng(0).choice(text.size, DUMP_GFA_MAX, replace=False))]
+    np.save(os.path.join(directory, "gfa.npy"), text.astype(np.float32))
+    np.save(os.path.join(directory, "gfa_size.npy"), np.array([len(gfa)], dtype=np.float64))
+    np.save(os.path.join(directory, "graph_counts.npy"), np.array(counts, dtype=np.float64))
 
 
 def measured_peak():
@@ -318,6 +339,9 @@ def run_gpu(args):
         parity = {"sha256": sha, "golden": golden, "golden_key": golden_key, "ok": bool(golden) and sha == golden and sha2 == golden,
                   "checked": "last step of the resident-input loop and of the host-buffer (e2e) loop" + ("" if world == 1 else "; the file is rank 0's H/S/L text followed by the ranks' P lines")}
         gfa = file1
+        if args.dump_outputs:      # the last step of the host-buffer loop: the call a user makes
+            c = last2[0].counts()
+            dump_outputs(args.dump_outputs, file2, [c.n_kmers, c.n_unitigs, c.n_links, c.total_length])
     if rank != 0:
         if world > 1:
             dist.destroy_process_group()
@@ -491,6 +515,8 @@ def run_reference(args):
             times.append(dt)
         if len(times) >= args.steps or (times and sum(times) + dt > budget_s):
             break
+    if args.dump_outputs:
+        dump_outputs(args.dump_outputs, gfa.encode(), [st.n_kmers, st.unitigs_after, st.links_after, st.length_after])
     total = sum(times)
     v = round(n_bases * len(times) / total / 1e6, 4)
     golden = golden_for(golden_key)
@@ -520,7 +546,10 @@ def main():
     ap.add_argument("--k", type=int, default=51)
     ap.add_argument("--no-cpu-baseline", action="store_true", help="skip the CPU oracle leg and the CLI runs (profiling and A/B runs)")
     ap.add_argument("--no-cli-wall", action="store_true", help="skip the two `autocycler compress` process runs that report the CLI's wall clock")
+    ap.add_argument("--dump-outputs", metavar="DIR", default=None, help="write what the last timed step returned to DIR/<name>.npy (float32 / float64)")
     args = ap.parse_args()
+    if args.steps < 1 or args.warmup < 0:
+        ap.error("--steps must be at least 1 and --warmup at least 0")
     args.no_cli_wall = args.no_cli_wall or args.no_cpu_baseline          # profiling and A/B runs: the device path only
     if args.impl == "reference":
         run_reference(args)

@@ -1,7 +1,10 @@
 """ctypes loader for the CPU oracle (oracle/liboracle.so) — test infrastructure only."""
+import atexit
 import ctypes as C
 import os
+import shutil
 import subprocess
+import tempfile
 
 ROOT = os.path.dirname(os.path.dirname(os.path.abspath(__file__)))
 ORACLE_DIR = os.path.join(ROOT, "oracle")
@@ -30,14 +33,17 @@ def build():
 
 
 def use_native():
-    """bench.py's CPU arm: build the oracle for THIS machine (-O3 -march=native, oracle/_native/) and use that library.
-    Must be called before the first oracle call of the process.  Returns the compiler flags in use."""
+    """bench.py's CPU arm: build the oracle for THIS machine (-O3 -march=native) in a temporary directory, removed at exit, and use
+    that library; the tree may be read-only.  Must be called before the first oracle call of the process.  Returns the compiler flags
+    in use."""
     global _path, build_flags
     assert _lib is None, "use_native() must precede the first oracle call"
+    out = tempfile.mkdtemp(prefix="autocycler_oracle_native_")
+    atexit.register(shutil.rmtree, out, True)
     try:
-        subprocess.run(["make", "-s", "-C", ORACLE_DIR, "native"], check=True, capture_output=True, timeout=600)
-        _path = os.path.join(ORACLE_DIR, "_native", "liboracle.so")
-        build_flags = open(os.path.join(ORACLE_DIR, "_native", "flags.txt")).read().strip()
+        subprocess.run(["make", "-s", "-C", ORACLE_DIR, "native", f"NATIVE_DIR={out}"], check=True, capture_output=True, timeout=600)
+        _path = os.path.join(out, "liboracle.so")
+        build_flags = open(os.path.join(out, "flags.txt")).read().strip()
     except Exception as e:      # no compiler on this machine: the shipped portable build is used, and the line says so
         build_flags += f" [native build failed: {type(e).__name__}]"
     return build_flags

@@ -15,8 +15,20 @@ def run(env=None, *args):
                           env={**os.environ, **(env or {})}, timeout=900, cwd=ROOT)
 
 
-def test_reference_arm_line():
-    r = run(None, "--steps", "2", "--warmup", "1", "--workload", "cfg1")      # the default (full cfg2) takes minutes per pass on one core
+def check_dump(directory, golden_key):
+    """--dump-outputs: the last timed step's GFA (cfg1's fits whole) and graph counts, against the oracle's committed values."""
+    import hashlib
+    import numpy as np
+    g = json.load(open(os.path.join(ROOT, "tests", "golden", "config_goldens.json")))[golden_key]
+    gfa = np.load(os.path.join(directory, "gfa.npy"))
+    assert gfa.dtype == np.float32 and hashlib.sha256(gfa.astype(np.uint8).tobytes()).hexdigest() == g["sha256"]
+    assert np.load(os.path.join(directory, "gfa_size.npy")).tolist() == [g["gfa_bytes"]]
+    counts = np.load(os.path.join(directory, "graph_counts.npy"))
+    assert counts.dtype == np.float64 and counts[:3].tolist() == [g["n_kmers"], g["unitigs_after"], g["links_after"]]
+
+
+def test_reference_arm_line(tmp_path):
+    r = run(None, "--steps", "2", "--warmup", "1", "--workload", "cfg1", "--dump-outputs", str(tmp_path / "out"))      # the default (full cfg2) takes minutes per pass on one core
     assert r.returncode == 0, r.stderr[-2000:]
     lines = [l for l in r.stdout.splitlines() if l.startswith("{")]
     assert len(lines) == 1
@@ -31,6 +43,7 @@ def test_reference_arm_line():
     assert "-march=native" in d["cpu_baseline"]["build"] and d["cpu_baseline"]["host_cores"] >= 1
     assert "workload" in d["config"] and "sample" in d["config"] and d["config"]["input_bases"] == 299982
     assert d["steps_timed"] == 2 and d["parity"]["ok"] is True and d["parity"]["golden_key"] == "cfg1_k51"      # the timed output is the committed oracle output
+    check_dump(tmp_path / "out", "cfg1_k51")
 
 
 def test_workload_selection_matches_the_committed_goldens():
@@ -52,11 +65,11 @@ def test_reference_arm_other_ranks_do_nothing():
 
 
 @pytest.mark.gpu
-def test_b200_arm_line():
+def test_b200_arm_line(tmp_path):
     """The B200 arm on the smallest BASELINE config (a second or two on the GPU): one JSON line with the driver's keys, the timed output
     equal to the oracle's committed hash, kernels of this library counted, the roofline entry for the insert kernel timed on its own."""
-    r = subprocess.run([sys.executable, os.path.join(ROOT, "bench.py"), "--workload", "cfg1", "--steps", "3", "--warmup", "3", "--no-cpu-baseline"],
-                       capture_output=True, text=True, timeout=600, cwd=ROOT)
+    r = subprocess.run([sys.executable, os.path.join(ROOT, "bench.py"), "--workload", "cfg1", "--steps", "3", "--warmup", "3", "--no-cpu-baseline",
+                        "--dump-outputs", str(tmp_path / "out")], capture_output=True, text=True, timeout=600, cwd=ROOT)
     assert r.returncode == 0, r.stderr[-2000:]
     lines = [l for l in r.stdout.splitlines() if l.startswith("{")]
     assert len(lines) == 1
@@ -71,3 +84,4 @@ def test_b200_arm_line():
     rf = d["roofline"]
     assert rf["bound"] == "hbm" and rf["unit"] == "GB/s" and 0 < rf["frac"] < 1 and abs(rf["frac"] - rf["achieved"] / rf["peak"]) < 1e-3
     assert 0 < rf["kernel_ms"] <= d["stage_ms"]["insert"] + 1e-3 and d["stage_ms"]["host_simplify"] == 0 and d["stage_ms"]["host_gfa"] == 0
+    check_dump(tmp_path / "out", "cfg1_k51")
